@@ -173,13 +173,14 @@ def fill_synthetic(cache: RefStaticCache, ctx):
     cache.stream_len = [cache.sink + cache.recent] * len(cache.n_full)
 
 
-def run(model, n_full_list, sink, recent, ctx, prefill_ctx, chunk, vocab, decode_steps=10, do_prefill=True):
+def run(model, n_full_list, sink, recent, ctx, prefill_ctx, chunk, vocab, decode_steps=10, decode_warmup=3,
+        do_prefill=True):
     """-> dict with the reference arm's end-to-end decode tokens/s at `ctx` and prefill tokens/s at `prefill_ctx`."""
     dev = next(model.parameters()).device
     r = RefRunner(model, n_full_list, sink, recent, max(ctx, prefill_ctx) + 8)
     res = {"what": "duo_attn/patch/llama.py:309-434 + static_kv_cache.py restated with the installed flash_attn_func "
                    f"(token-major caches, 2 FA2 calls + cat, compaction copies), eager; rope: {r.rope}; rmsnorm: {r.norm}",
-           "protocol": "eval/efficiency/utils.py bench_func (CUDA events); decode: 3 warm-up + "
+           "protocol": f"eval/efficiency/utils.py bench_func (CUDA events); decode: {decode_warmup} warm-up + "
                        f"{decode_steps} steps with evict_last(1); prefill: 1 rep after a one-chunk warm-up"}
     g = torch.Generator().manual_seed(1)
     if do_prefill:
@@ -203,7 +204,7 @@ def run(model, n_full_list, sink, recent, ctx, prefill_ctx, chunk, vocab, decode
         r.forward(tok)
         r.cache.evict_last(1)
 
-    for _ in range(3):
+    for _ in range(decode_warmup):
         step()
     torch.cuda.synchronize()
     e0, e1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)

@@ -16,6 +16,11 @@ layer, fused one-shot all-reduce for the MLP), reached from the prefill layout b
 -> "strong".
 
   python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--ctx 1048576] [--prefill-ctx 131072]
+                  [--dump-outputs DIR]
+
+--dump-outputs DIR writes the logits the timed prefill and decode returned in their last repetition / step as
+DIR/prefill_logits.npy and DIR/decode_logits.npy (float32).  Weights, token ids and the synthetic cache come from fixed
+seeds, so two builds run with the same arguments can be compared output for output.
 """
 from __future__ import annotations
 
@@ -93,7 +98,14 @@ def parse():
                          "gpurun_out/profile_step_n<N>.txt; never used for a bench value")
     ap.add_argument("--head-tp-decode", action="store_true",
                     help="N > 1: decode head-parallel like the reference's TP rule instead of sequence-sharded (A/B)")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="after the timed regions: write the logits of the last timed prefill and decode step to DIR "
+                         "(--impl ours only)")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl != "ours":
+        ap.error("--dump-outputs needs --impl ours: the reference arm extrapolates timings and returns no outputs")
     if args.pattern is None:
         args.pattern = ARCHS[args.arch][1]
     return args
@@ -183,8 +195,10 @@ def run_reference(args):
     if rank != 0:
         return
     mask, sp = head_pattern(args.pattern, args.sparsity)
+    for _ in range(args.warmup):
+        cpu_reference_sample(args.ctx, mask)
     vals = []
-    for _ in range(max(1, min(args.steps, 5))):
+    for _ in range(args.steps):  # one sample = one extrapolated decode step
         vals.append(cpu_reference_sample(args.ctx, mask))
     best = sorted(vals, key=lambda r: r["tok_s"])[len(vals) // 2]  # median of the samples, not the best
     line = {
@@ -375,6 +389,7 @@ def main():
         return float(t.item())
 
     result = {}
+    dumps = {}  # --dump-outputs: name -> host tensor
     launches = 0
     # ------------------------------------------------------------------ prefill @128K
     seq_decode = world > 1 and args.kv_format == "bf16" and not args.head_tp_decode
@@ -392,7 +407,7 @@ def main():
                 chunk = ids_host[:, i : i + args.chunk].to(dev, non_blocking=True)
                 out = model(input_ids=chunk, past_key_values=cache, use_cache=True)
             tok = out.logits[:, -1, :].argmax(-1)
-            return int(tok.item()) if e2e else tok
+            return (int(tok.item()) if e2e else tok), out.logits
 
         with torch.no_grad():
             prefill_once(False)  # warm-up (cuBLAS heuristics, TMA descriptors, allocator)
@@ -405,7 +420,7 @@ def main():
                 e0, e1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
                 torch.cuda.nvtx.range_push("timed_prefill")
                 e0.record()
-                prefill_once(True)  # host ids in, host token out: this IS the end-to-end call
+                _, logits = prefill_once(True)  # host ids in, host token out: this IS the end-to-end call
                 e1.record()
                 barrier()
                 torch.cuda.nvtx.range_pop()
@@ -413,6 +428,8 @@ def main():
                 attn_times.append(sum(a.elapsed_time(b) for a, b in cache.profile_events))
             cache.profile_events = None
             launches_prefill = cache.launch_count + ops.LAUNCHES - c0
+            if args.dump_outputs:
+                dumps["prefill_logits"] = logits.float().cpu()
         best = min(range(len(times)), key=lambda i: times[i])
         ms = times[best]
         fl = prefill_flops(mask, args.prefill_ctx, args.chunk, G=32 // mask.shape[1])
@@ -456,6 +473,8 @@ def main():
                 result["prefill"][key] = max_over_ranks(e0.elapsed_time(e1))
         if args.prefill_only:
             if rank == 0:
+                if args.dump_outputs:
+                    write_dumps(args.dump_outputs, dumps)
                 print(json.dumps({"prefill_only": True, "n_gpus": world, "tp_pipeline_blocks": args.tp_pipeline_blocks,
                                   **result}), flush=True)
             dist.barrier()
@@ -473,12 +492,13 @@ def main():
 
     def decode_step_resident():
         if graph is not None:
-            graph.step(tok_dev)
+            logits = graph.step(tok_dev)
         else:
-            model(input_ids=tok_dev, past_key_values=cache, use_cache=True)
+            logits = model(input_ids=tok_dev, past_key_values=cache, use_cache=True).logits
         cache.evict_last(1)
         if graph is not None:
             graph.resync()
+        return logits
 
     def decode_step_e2e():
         if graph is not None:
@@ -519,11 +539,13 @@ def main():
         torch.cuda.nvtx.range_push("timed_decode")
         e0.record()
         for _ in range(args.steps):
-            decode_step_resident()
+            logits = decode_step_resident()
         e1.record()
         barrier()
         torch.cuda.nvtx.range_pop()
         ms_total = max_over_ranks(e0.elapsed_time(e1))
+        if args.dump_outputs:  # copied now: the graph's output buffer is overwritten by the next replay
+            dumps["decode_logits"] = logits.float().cpu()
         launches = cache.launch_count + ops.LAUNCHES - c0
         # --- e2e: host token in, host token out, every step
         for _ in range(2):
@@ -595,7 +617,8 @@ def main():
             from baseline import fa2_restated
 
             ref = fa2_restated.run(model, [int(x) for x in mask.sum(1)], SINK, RECENT, args.ctx, args.prefill_ctx,
-                                   args.chunk, vocab, do_prefill=not args.no_prefill)
+                                   args.chunk, vocab, decode_steps=args.steps, decode_warmup=max(3, args.warmup),
+                                   do_prefill=not args.no_prefill)
             ref["decode"]["ours_over_reference"] = line["e2e"]["value"] / ref["decode"]["value"]
             if "prefill" in ref and "prefill" in line:
                 ref["prefill"]["ours_over_reference"] = line["prefill"]["value"] / ref["prefill"]["value"]
@@ -615,6 +638,8 @@ def main():
                                           "KV head + 1 layer of linears, extrapolated to 128+128 heads x 32 layers",
                                 "t_full_head_s": cb["t_full_head_s"]}
     if rank == 0:
+        if args.dump_outputs:
+            write_dumps(args.dump_outputs, dumps)
         print(json.dumps(line), flush=True)
     if world > 1:
         # NCCL communicators captured inside the CUDA graph make destroy_process_group() hang: synchronise,
@@ -771,6 +796,14 @@ def per_step_launches(cache, ops, model, tok_dev):
     cache.dev_state = ds
     cache.sync_device_state()
     return cache.launch_count + ops.LAUNCHES - c0
+
+
+def write_dumps(out_dir, dumps):
+    import numpy as np
+
+    os.makedirs(out_dir, exist_ok=True)
+    for name, t in dumps.items():
+        np.save(os.path.join(out_dir, f"{name}.npy"), t.numpy().astype(np.float32))
 
 
 def ms_step_guess(ms_total, steps):

@@ -1,7 +1,8 @@
 """Compile the reference's ONLY native source, demo/quantize_int4.cu, where it lies under
 /root/reference, into oracle/_ref/ (git-ignored, travels to the GPU box).  TEST INFRASTRUCTURE ONLY:
-the resulting module is the real reference implementation of INT4 quantise/dequantise (kernels K1/K2) and
-is used by tests/test_gpu_int4.py to pin both the NumPy oracle and the product kernels.
+the resulting module is the real reference implementation of INT4 quantise/dequantise (kernels K1/K2);
+``tests/golden/make_golden.py int4-kernels`` runs it to write the fixture that pins both the NumPy oracle and the
+product kernels.
 
 The reference JIT-builds this file with ``torch.utils.cpp_extension.load(extra_cuda_cflags=
 ["--use_fast_math"])`` (demo/int4_kv.py:46-56); we do the same ahead of time for sm_100a.  No reference

@@ -5,6 +5,10 @@ need it):
 
     python tests/golden/make_golden.py
 
+``int4_ref_kernels.npz`` comes from the reference's compiled INT4 kernels instead, on a GPU (``make_int4_kernel_fixture``):
+
+    python oracle/build_ref.py && python tests/golden/make_golden.py int4-kernels [OUT_DIR]
+
 How the reference is made importable here (SURVEY.md §8c says it is not, as-is):
   * transformers 5.5 no longer re-exports ``List / Union / CrossEntropyLoss`` from modeling_llama — we add
     those three names to the real module before importing ``duo_attn.patch.llama``;
@@ -288,12 +292,44 @@ def make_training_mask_fixtures(GC):
     print("wrote training masks", len(GC.TRAIN_MASK_CASES))
 
 
+def make_int4_kernel_fixture(GC, out_dir):
+    """The reference's INT4 quantise (K1) and dequantise (K2) kernels of demo/quantize_int4.cu, built with its own flags
+    (--use_fast_math) into oracle/_ref/ by oracle/build_ref.py, on GC.make_int4_kernel_input().  Needs a GPU.  K1's
+    packed codes, scales and zeros are kept for every row; K2's dequantisation of them (614 KB of fp16) is kept as the
+    SHA-256 of its bytes, which the tests compare bit for bit."""
+    import hashlib
+
+    from oracle import build_ref
+
+    ref = build_ref.load_module()
+    assert ref is not None, "oracle/_ref/ not built: python oracle/build_ref.py"
+    x = GC.make_int4_kernel_input()
+    rows_n = x.size // 128
+    dev = torch.device("cuda:0")
+    xt = torch.from_numpy(x).to(dev)
+    qp = torch.empty(*x.shape[:-1], 64, dtype=torch.uint8, device=dev)
+    sc = torch.empty(*x.shape[:-1], 1, dtype=torch.float16, device=dev)
+    zp = torch.empty(*x.shape[:-1], 1, dtype=torch.float16, device=dev)
+    ref.quantize_int4_with_zero_point_per_group(xt, qp, sc, zp, 128)
+    buf = torch.empty(rows_n * 128, dtype=torch.float16, device=dev)
+    ref.dequantize_int4_with_zero_point_per_group(qp.view(-1, 64), sc, zp, 128, buf, rows_n)
+    torch.cuda.synchronize()
+    np.savez_compressed(
+        os.path.join(out_dir, "int4_ref_kernels.npz"),
+        packed=qp.view(-1, 64).cpu().numpy(), scale=sc.view(-1).cpu().numpy(), zero=zp.view(-1).cpu().numpy(),
+        dequant_sha256=np.str_(hashlib.sha256(buf.view(-1, 128).cpu().numpy().tobytes()).hexdigest()),
+        checksum=np.float64(np.abs(x.astype(np.float64)).sum()))
+    print("wrote int4_ref_kernels,", rows_n, "rows")
+
+
 def main():
     from oracle import duo_oracle as O
     import golden_cases as GC
 
     if sys.argv[1:] == ["masks"]:
         return make_training_mask_fixtures(GC)
+    if sys.argv[1:2] == ["int4-kernels"]:
+        return make_int4_kernel_fixture(GC, sys.argv[2] if len(sys.argv) > 2 else HERE)
 
     ref_llama, ref_mistral, ref_putils, ref_utils = import_reference()
     assert ref_llama.__file__.startswith(REF), ref_llama.__file__

@@ -76,6 +76,13 @@ def int4_checksum(chunks):
     return float(sum(float(t.double().abs().sum()) for c in chunks for t in c))
 
 
+def make_int4_kernel_input():
+    """[2, 300, 4, 128] fp16 for the INT4 quantise / dequantise kernels: 2400 groups of 128 whose magnitudes span two
+    decades."""
+    rng = np.random.RandomState(2)
+    return (rng.randn(2, 300, 4, D) * rng.uniform(0.05, 5, size=(2, 300, 4, 1))).astype(np.float16)
+
+
 # Model-level drivers (tuple_kv_cache.py / static_kv_cache.py patched ForCausalLM forwards + enable_* functions)
 MODEL_CASES = [
     dict(name="llama_tuple", kind="llama", path="tuple", gates=[[1.0, 0.0], [0.0, 1.0]], sink=4, recent=6,

@@ -1,11 +1,14 @@
 """RoPE + append + ring commit + INT4 quantise kernels vs torch / the oracles / the reference's own
-kernels (oracle/_ref, compiled from /root/reference/demo/quantize_int4.cu)."""
+kernels (demo/quantize_int4.cu; their outputs are stored in tests/golden/int4_ref_kernels.npz)."""
 import ctypes as C
+import hashlib
+import os
 
 import numpy as np
 import pytest
 import torch
 
+import golden_cases as GC
 from duo_attention_b200 import _C
 from duo_attention_b200.kv_cache import DuoKVCache, ring_slot
 from oracle import duo_oracle as O
@@ -148,40 +151,30 @@ def test_dequant_matches_numpy_oracle_bit_exact():
 
 
 def test_quant_dequant_vs_reference_kernels_compiled_from_source():
-    """oracle/_ref = the reference's demo/quantize_int4.cu built with its own flags (--use_fast_math).
+    """The reference's demo/quantize_int4.cu built with its own flags (--use_fast_math); its outputs on this input
+    are the fixture (tests/golden/make_golden.py int4-kernels): codes, scales and zeros of every row, and the SHA-256
+    of its dequantisation of them.
     scale/zero must be bit-exact; codes may differ by one only on (near-)exact .5 ties because the
     reference's fast-math division is approximate; dequantise is bit-exact."""
-    from oracle import build_ref
-
-    ref = build_ref.load_module()
-    if ref is None:
-        pytest.skip("oracle/_ref not built (needs /root/reference at build time)")
-    rng = np.random.RandomState(2)
-    x = (rng.randn(2, 300, 4, 128) * rng.uniform(0.05, 5, size=(2, 300, 4, 1))).astype(np.float16)
-    xt = torch.from_numpy(x).to(dev)
-    qp = torch.empty(2, 300, 4, 64, dtype=torch.uint8, device=dev)
-    sc = torch.empty(2, 300, 4, 1, dtype=torch.float16, device=dev)
-    zp = torch.empty(2, 300, 4, 1, dtype=torch.float16, device=dev)
-    ref.quantize_int4_with_zero_point_per_group(xt, qp, sc, zp, 128)
-    torch.cuda.synchronize()
-    p, s, z = _quant_gpu(xt)
-    assert torch.equal(s.view(-1), sc.view(-1)) and torch.equal(z.view(-1), zp.view(-1))
+    fx = np.load(os.path.join(os.path.dirname(os.path.abspath(__file__)), "golden", "int4_ref_kernels.npz"))
+    x = GC.make_int4_kernel_input()
+    assert abs(np.abs(x.astype(np.float64)).sum() - float(fx["checksum"])) < 1e-9 * float(fx["checksum"]), "RNG drift"
+    p, s, z = _quant_gpu(torch.from_numpy(x))
+    assert np.array_equal(s.cpu().numpy(), fx["scale"]) and np.array_equal(z.cpu().numpy(), fx["zero"])
     mine = Q.unpack_codes(p.cpu().numpy()).astype(np.int32).reshape(-1)
-    theirs = Q.unpack_codes(qp.cpu().numpy().reshape(-1, 64)).astype(np.int32).reshape(-1)
+    theirs = Q.unpack_codes(fx["packed"]).astype(np.int32).reshape(-1)
     diff = np.abs(mine - theirs)
     assert diff.max() <= 1 and (diff != 0).mean() < 2e-3, (diff.max(), (diff != 0).mean())
     # where they differ the true quotient sits on a rounding tie
     po, so, zo = Q.quantize_int4(x.reshape(-1, 128))
     assert np.array_equal(Q.unpack_codes(po).reshape(-1), mine)
     # K2: dequantise their packed data with both
-    buf = torch.empty(2 * 300 * 4 * 128, dtype=torch.float16, device=dev)
-    ref.dequantize_int4_with_zero_point_per_group(qp.view(-1, 64), sc, zp, 128, buf, 2 * 300 * 4)
-    torch.cuda.synchronize()
-    mine_d = torch.empty(2 * 300 * 4, 128, dtype=torch.float16, device=dev)
+    n = fx["packed"].shape[0]
+    qp, sc, zp = (torch.from_numpy(fx[k]).to(dev).contiguous() for k in ("packed", "scale", "zero"))
+    mine_d = torch.empty(n, 128, dtype=torch.float16, device=dev)
     lib = _C.load()
-    _C.check(lib.duo_dequant_int4(qp.data_ptr(), sc.data_ptr(), zp.data_ptr(), 2 * 300 * 4, mine_d.data_ptr(),
+    _C.check(lib.duo_dequant_int4(qp.data_ptr(), sc.data_ptr(), zp.data_ptr(), n, mine_d.data_ptr(),
                                   torch.cuda.current_stream().cuda_stream))
-    assert torch.equal(mine_d.view(-1), buf)
-    assert np.array_equal(buf.cpu().numpy().reshape(-1, 128),
-                          Q.dequantize_int4(qp.cpu().numpy().reshape(-1, 64), sc.cpu().numpy().reshape(-1, 1),
-                                            zp.cpu().numpy().reshape(-1, 1)))
+    oracle_d = Q.dequantize_int4(fx["packed"], fx["scale"].reshape(-1, 1), fx["zero"].reshape(-1, 1))
+    assert np.array_equal(mine_d.cpu().numpy(), oracle_d)
+    assert hashlib.sha256(oracle_d.tobytes()).hexdigest() == str(fx["dequant_sha256"])

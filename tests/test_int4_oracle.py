@@ -1,5 +1,5 @@
-"""Properties of the NumPy INT4 oracle (restating demo/quantize_int4.cu); the GPU tests pin it against
-the reference kernels compiled from source (oracle/_ref) on the B200 box."""
+"""Properties of the NumPy INT4 oracle (restating demo/quantize_int4.cu); tests/test_gpu_kv_ops.py pins it against
+the reference kernels' stored outputs (tests/golden/int4_ref_kernels.npz)."""
 import numpy as np
 
 from oracle import int4_oracle as Q
